@@ -5,7 +5,7 @@ backward) on synthetic OD tensors, on N GPUs of one node.
     python bench.py --gpus 1 --steps 10 --warmup 3
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W [--shard batch|row|k]
-    python bench.py --impl reference --steps K --warmup W        # CPU arm: the unmodified reference from baseline/_ref
+    python bench.py --impl reference --steps K --warmup W        # CPU arm: the unmodified reference from oracle/_ref
 
 Workload (BASELINE.json metric "OD-cells/sec (B*T*N^2) 2D-GCN fwd+bwd at N=1000,K=3"): `--workload headline` = N=1000
 nodes, K=3 supports, T=12, hidden 32, M=2 branches (static + dynamic graph), 3 BDGCN layers per branch, batch 8 per GPU
@@ -37,7 +37,7 @@ if ROOT not in sys.path:
 
 METRIC = "OD-cells/sec (B*T*N^2), MPGCN hot path fwd+bwd"
 UNIT = "OD-cells/s"
-REF_DIR = os.path.join(ROOT, "baseline", "_ref")
+REF_DIR = os.path.join(ROOT, "oracle", "_ref")
 
 WORKLOADS = {          # name: (N, K, T, batch per GPU)   -- BASELINE.json configs / SURVEY.md section 8(d)
     "headline": (1000, 3, 12, 8),
@@ -71,7 +71,12 @@ def parse():
     ap.add_argument("--no-gpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--profile", action="store_true", help="under ncu: honour --warmup < 3, skip the e2e / CPU / library arms (numbers are not bench values)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (loss, prediction, parameter gradients; rank 0's) "
+                         "as DIR/<name>.npy in float32, at most 64 MB in all")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     N, K, T, B = WORKLOADS[a.workload]
     a.nodes = a.nodes or N
     a.supports = a.supports or K
@@ -143,12 +148,12 @@ class ClockSampler:
 
 
 # ------------------------------------------------------------------------------------------------
-# the reference (unmodified, from baseline/_ref) or -- only where that is absent -- its torch port
+# the reference (unmodified, from oracle/_ref) or -- only where that is absent -- its torch port
 # ------------------------------------------------------------------------------------------------
 def load_reference_impl():
     """-> (module-like object with BDGCN and MPGCN classes, kind).  kind "reference": the unmodified classes of
-    underdoc-wang/MPGCN imported from baseline/_ref (baseline/install_ref.py put them there; the directory travels to the
-    GPU box but is not tracked); "port": oracle/torch_port.py, a torch restatement of the reference's execution order."""
+    underdoc-wang/MPGCN imported from oracle/_ref (oracle/install_ref.py put them there; the directory is not tracked);
+    "port": oracle/torch_port.py, a torch restatement of the reference's execution order."""
     f = os.path.join(REF_DIR, "MPGCN.py")
     if os.path.isfile(f):
         spec = importlib.util.spec_from_file_location("_reference_MPGCN", f)      # private name: the repo's MPGCN.py shim cannot shadow it
@@ -231,7 +236,7 @@ class CpuArm:
     def describe(self):
         a = self.a
         return (f"1/6 of one B=1 model step at full size: one BDGCN layer fwd+bwd (N={a.nodes}, K={a.supports}, C=H={a.hidden}; "
-                f"{'unmodified reference class from baseline/_ref' if self.kind == 'reference' else 'torch port of the reference order'}; static / dynamic "
+                f"{'unmodified reference class from oracle/_ref' if self.kind == 'reference' else 'torch port of the reference order'}; static / dynamic "
                 f"supports alternate) on {self.cores} threads + nn.LSTM fwd+bwd over {self.cells} of {a.nodes ** 2} cells, T={a.obs}, on "
                 f"{self.lstm_threads} threads (fastest of a probe); credited T*N*N/6 OD cells; no size extrapolation")
 
@@ -310,6 +315,30 @@ def gpu_library_baseline(a, dev):
 # ------------------------------------------------------------------------------------------------
 # GPU arm
 # ------------------------------------------------------------------------------------------------
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, model, loss, y_pred):
+    """Write what a training step computed -- loss.npy, y_pred.npy and grad.<parameter>.npy -- in float32, so that two builds
+    run with the same arguments (hence the same seeded inputs and weights) can be compared output for output.  A prediction
+    that does not fit in what is left of DUMP_BYTES is written as y_pred_sample.npy: the elements at a fixed, seeded set of
+    flat indices, the same for every run of the same shape."""
+    import numpy as np
+    import torch
+    arrays = {"loss": loss}
+    arrays.update(("grad." + n, p.grad) for n, p in model.named_parameters() if p.grad is not None)
+    left = DUMP_BYTES - 4 * sum(t.numel() for t in arrays.values())
+    flat = y_pred.reshape(-1)
+    if 4 * flat.numel() <= left:
+        arrays["y_pred"] = y_pred
+    else:
+        idx = np.unique(np.random.default_rng(0).integers(0, flat.numel(), left // 4))
+        arrays["y_pred_sample"] = flat[torch.from_numpy(idx).to(flat.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def run_ours(a):
     import torch
     import torch.distributed as dist
@@ -367,18 +396,20 @@ def run_ours(a):
         fwd = lambda x, go, gd: model(x_seq=x, G_list=[G_static, (go, gd)])
 
     def step(x, y, go, gd):
+        """-> (loss, prediction), detached: holding them keeps no autograd graph alive"""
         for p in params:
             p.grad = None
+        y_pred = fwd(x, go, gd)
         if sharded:
-            loss = mshard.sharded_mse_loss(plan, fwd(x, go, gd), y)
+            loss = mshard.sharded_mse_loss(plan, y_pred, y)
             loss.backward()
             # every rank holds partial parameter gradients of its group's samples: sum inside a group, mean over the groups
             mshard.allreduce_sum_gradients(params, plan, model, over_world=n_groups > 1, scale=1.0 / n_groups)
         else:
-            loss = crit(fwd(x, go, gd), y)
+            loss = crit(y_pred, y)
             loss.backward()
             mdist.allreduce_mean_gradients(params)      # the only exchange step of the batch shard (no-op for one rank)
-        return loss
+        return loss.detach(), y_pred.detach()
 
     def sync_all():
         if world > 1:
@@ -396,7 +427,7 @@ def run_ours(a):
     x, y, go, gd = (t.to(dev) for t in hosts)
     n_warm = a.warmup if a.profile else max(3, a.warmup)
     for _ in range(n_warm):
-        step(x, y, go, gd)
+        last = step(x, y, go, gd)         # kept like the timed steps' results, so the timed region allocates nothing new
     sync_all()
     lib.mpgcn_profile_reset()
     lib.mpgcn_profile_enable(1)
@@ -407,7 +438,7 @@ def run_ours(a):
     sync_all()
     e0.record()
     for _ in range(a.steps):
-        step(x, y, go, gd)
+        last = step(x, y, go, gd)
     e1.record()
     sync_all()
     ms = max_over_ranks(e0.elapsed_time(e1))
@@ -418,6 +449,9 @@ def run_ours(a):
     samples_per_step = B if sharded else world * B
     cells_per_step = samples_per_step * T * N * N
     value = cells_per_step / (ms_per_step * 1e-3)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, model, *last)
+    del last
 
     # ---- end-to-end arm: host buffers in, loss out, every step -----------------------------------
     e2e = None
@@ -447,7 +481,7 @@ def run_ours(a):
                     b.record_stream(torch.cuda.current_stream())
                 if k + 1 < n:
                     nxt = stage()
-                loss = step(*bufs)
+                loss, _ = step(*bufs)
                 losses.append(float(loss.item()))            # device -> host read of the loss, every step
             return losses
 

@@ -24,6 +24,9 @@ import torch
 
 REF = os.environ.get("MPGCN_REFERENCE_DIR", "/root/reference")
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
+ROOT = os.path.dirname(os.path.dirname(OUT))
+if ROOT not in sys.path:
+    sys.path.insert(0, ROOT)
 
 
 def _load_ref(name):
@@ -292,6 +295,51 @@ def gen_dyn(ref_data):
         print("wrote", name, o_g.shape, "nan:", int(np.isnan(o_g).sum()), int(np.isnan(d_g).sum()))
 
 
+# The trainer-style horizon loop of tests/test_trainer_dropin.py (Model_Trainer.py:157-165) on the reference model.  Inputs come
+# from seeds alone (`rollout_case_inputs`) and the weights are the default init under torch.manual_seed(seed) -- the same for
+# the reference class and the engine's drop-in; checksums of both are stored and asserted by the test -- so only the
+# reference's prediction is kept.
+ROLLOUT = dict(N=47, K=3, T=7, B=4, pred=5, seed=3)
+
+
+def rollout_model_kwargs():
+    return dict(M=2, K=ROLLOUT["K"], input_dim=1, lstm_hidden_dim=32, lstm_num_layers=1, gcn_hidden_dim=32, gcn_num_layers=3,
+                num_nodes=ROLLOUT["N"], user_bias=True, activation=torch.nn.ReLU)
+
+
+def rollout_case_inputs():
+    """(x [B,T,N,N,1], G [K,N,N], G_o [B,K,N,N], G_d [B,K,N,N]) of the rollout fixture: random-walk supports of U[0,1)
+    adjacencies through the oracle's adj_process (pinned to the reference by the adj_* fixtures)."""
+    from oracle import mpgcn_oracle as orc
+    N, K, T, B = (ROLLOUT[k] for k in "NKTB")
+    rng = np.random.default_rng(1)
+    x = (rng.random((B, T, N, N, 1)) * 6).astype(np.float32)
+    sup = lambda b: orc.adj_process(rng.random((max(b, 1), N, N)).astype(np.float32), "random_walk_diffusion", K - 1).astype(np.float32)
+    G, go, gd = sup(0)[0], sup(B), sup(B)
+    return x, G, go, gd
+
+
+def horizon_loop(model, x, G_list, pred):
+    """The reference trainer's autoregressive test loop (Model_Trainer.py:157-165)."""
+    y_pred, cur = [], x
+    with torch.no_grad():
+        for _ in range(pred):
+            step = model(x_seq=cur, G_list=G_list)
+            cur = torch.cat([cur[:, 1:, :, :, :], step], dim=1)
+            y_pred.append(step)
+    return torch.cat(y_pred, dim=1)
+
+
+def gen_rollout(ref_mpgcn):
+    torch.manual_seed(ROLLOUT["seed"])
+    model = ref_mpgcn.MPGCN(**rollout_model_kwargs()).eval()
+    x, G, go, gd = (torch.from_numpy(a) for a in rollout_case_inputs())
+    y = horizon_loop(model, x, [G, (go, gd)], ROLLOUT["pred"])
+    np.savez_compressed(os.path.join(OUT, "rollout_n47_k3_p5.npz"), y=_np(y), x_checksum=np.float64(x.double().sum()),
+                        param_sums=np.array([float(v.double().sum()) for v in model.state_dict().values()]))
+    print("wrote rollout_n47_k3_p5", tuple(y.shape))
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
     torch.set_num_threads(max(1, os.cpu_count() or 1))
@@ -313,6 +361,8 @@ def main():
         gen_adj(ref_gcn)
     if want("dyn"):
         gen_dyn(_load_ref("Data_Container_OD"))
+    if want("rollout"):
+        gen_rollout(ref_mpgcn)
 
 
 if __name__ == "__main__":

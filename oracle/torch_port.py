@@ -111,7 +111,7 @@ class PortBDGCN(torch.nn.Module):
 class PortMPGCN(torch.nn.Module):
     """The port's model: per branch nn.LSTM over B*N*N cells (zero state, last step) -> L x PortBDGCN -> Linear+ReLU, mean over
     branches (MPGCN.py:54-112), including the reference's materialisations (zero (h0, c0), the full lstm_out, stack + mean).
-    Used only where the real reference (baseline/_ref) is not available."""
+    Used only where the real reference (oracle/_ref) is not available."""
 
     def __init__(self, M, K, input_dim, lstm_hidden_dim, lstm_num_layers, gcn_hidden_dim, gcn_num_layers, num_nodes, user_bias,
                  activation=None):

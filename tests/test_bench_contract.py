@@ -1,5 +1,5 @@
 """bench.py's output contract, as far as it can be checked without a GPU: the reference arm (`--impl reference`) runs the unmodified
-reference from baseline/_ref (or the torch port) on a bounded sample and prints ONE JSON line with the keys the driver reads, with
+reference from oracle/_ref (or the torch port) on a bounded sample and prints ONE JSON line with the contract keys, with
 the same `config` the GPU arm would print for those arguments."""
 import json
 import os
@@ -30,7 +30,7 @@ def test_reference_arm_prints_one_json_line_with_the_contract_keys():
     import bench
     a = type("A", (), dict(nodes=60, supports=3, obs=4, batch=2, hidden=32, precision="fp16", shard="batch", row_ranks=0))()
     assert d["config"] == bench.workload_config(a, 1)
-    if os.path.isfile(os.path.join(ROOT, "baseline", "_ref", "MPGCN.py")):
+    if os.path.isfile(os.path.join(ROOT, "oracle", "_ref", "MPGCN.py")):
         assert cb["kind"] == "reference"
 
 

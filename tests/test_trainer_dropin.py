@@ -4,7 +4,8 @@
 The reference ships no data (Data_Container_OD.py:15,34 read `od_day20180101_20210228.npz` and `adjacency_matrix.npy`), so
 the tests write a synthetic pair of the right format (route (i) of SURVEY.md section 8(c)): a scipy sparse matrix whose
 dense form reshapes to (-1, 47, 47) with >= 425 day rows, and a [47, 47] adjacency.  The reference itself is imported from
-`baseline/_ref` (baseline/install_ref.py; untracked, travels to the GPU box); without it the tests skip.
+`oracle/_ref` (oracle/install_ref.py; untracked); without it the two trainer tests skip.  The rollout test compares with the
+reference's prediction stored in tests/golden/ and needs no reference.
 
   * CPU (`-m "not gpu"`): the stock reference runs one epoch on that data (`tools/run_main.py --stock -GPU cpu`) -- the data
     shim is what Main.py expects;
@@ -21,10 +22,10 @@ import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "baseline", "_ref")
+REF = os.path.join(ROOT, "oracle", "_ref")
 RUN_MAIN = os.path.join(ROOT, "tools", "run_main.py")
 
-needs_ref = pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "Main.py")), reason="baseline/_ref (the unmodified reference) is not installed")
+needs_ref = pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "Main.py")), reason="oracle/_ref (the unmodified reference) is not installed")
 
 
 def write_synthetic_data(dirname, days=430, N=47, seed=0):
@@ -114,56 +115,44 @@ def test_unchanged_trainer_trains_and_tests_on_the_engine(tmp_path):
         assert np.allclose(ve, vg, rtol=1e-3), (le, lg)
 
 
-@needs_ref
 @pytest.mark.gpu
 def test_graph_rollout_install_matches_eager_and_reference(tmp_path):
     """rollout.install(model): the trainer-style horizon loop (Model_Trainer.py:157-165) through the captured graph is
-    bit-identical to the eager loop, and both match the REFERENCE model's own loop (fp32 engine: <= 1e-4; fp16: <= 2e-3)."""
+    bit-identical to the eager loop, and both match the REFERENCE model's own loop (fp32 engine: <= 1e-4; fp16: <= 2e-3).
+    The reference's prediction is the golden fixture rollout_n47_k3_p5 (oracle/gen_golden.py); its inputs and weights are
+    regenerated here from the fixture's seeds and checked against the stored checksums."""
     import torch
-    from torch import nn
     if not torch.cuda.is_available():
         pytest.skip("no CUDA device")
-    import importlib.util
-    spec = importlib.util.spec_from_file_location("_ref_MPGCN_rollout", os.path.join(REF, "MPGCN.py"))
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
     sys.path.insert(0, ROOT)
     import MPGCN as shim
+    from conftest import load_golden
     from mpgcn_b200 import rollout
     from oracle import mpgcn_oracle as orc
+    from oracle.gen_golden import ROLLOUT, horizon_loop, rollout_case_inputs, rollout_model_kwargs
     dev = torch.device("cuda:0")
-    N, K, T, B, pred = 47, 3, 7, 4, 5
-    torch.manual_seed(3)
-    kw = dict(M=2, K=K, input_dim=1, lstm_hidden_dim=32, lstm_num_layers=1, gcn_hidden_dim=32, gcn_num_layers=3, num_nodes=N,
-              user_bias=True, activation=nn.ReLU)
-    ref_model = ref.MPGCN(**kw).eval()
-    rng = np.random.default_rng(1)
-    x = torch.from_numpy((rng.random((B, T, N, N, 1)) * 6).astype(np.float32))
-    sup = lambda b: torch.from_numpy(orc.adj_process(rng.random((max(b, 1), N, N)).astype(np.float32), "random_walk_diffusion", K - 1).astype(np.float32))
-    G, go, gd = sup(0)[0], sup(B), sup(B)
-
-    def horizon_loop(model, x, G_list):          # the reference's loop, Model_Trainer.py:157-165
-        y_pred, cur = [], x
-        with torch.no_grad():
-            for _ in range(pred):
-                step = model(x_seq=cur, G_list=G_list)
-                cur = torch.cat([cur[:, 1:, :, :, :], step], dim=1)
-                y_pred.append(step)
-        return torch.cat(y_pred, dim=1)
-
-    want = horizon_loop(ref_model, x, [G, (go, gd)]).numpy()
+    g = load_golden("rollout_n47_k3_p5")
+    kw = rollout_model_kwargs()
+    torch.manual_seed(ROLLOUT["seed"])
+    init = shim.MPGCN(**kw).state_dict()          # the reference class draws the same default init under this seed
+    np.testing.assert_allclose([float(v.double().sum()) for v in init.values()], g["param_sums"], rtol=1e-12,
+                               err_msg="the default init no longer matches the weights the fixture was made with")
+    x, G, go, gd = (torch.from_numpy(a) for a in rollout_case_inputs())
+    np.testing.assert_allclose(float(x.double().sum()), float(g["x_checksum"]), rtol=1e-12)
+    pred = ROLLOUT["pred"]
+    want = g["y"]
     for prec, tol in (("fp32", 1e-4), ("fp16", 2e-3)):
         model = shim.MPGCN(**kw)
-        model.load_state_dict(ref_model.state_dict())
+        model.load_state_dict(init)
         model = model.to(dev).eval()
         model.lstm_precision = prec
         for mod in model.modules():
             if isinstance(mod, shim.BDGCN):
                 mod.precision = prec
         G_list = [G.to(dev), (go.to(dev), gd.to(dev))]
-        eager = horizon_loop(model, x.to(dev), G_list)
+        eager = horizon_loop(model, x.to(dev), G_list, pred)
         rollout.install(model)
-        graphed = horizon_loop(model, x.to(dev), G_list)
+        graphed = horizon_loop(model, x.to(dev), G_list, pred)
         assert model.forward.captures == 1 and model.forward.replays == pred
         assert torch.equal(eager, graphed)
         rollout.uninstall(model)

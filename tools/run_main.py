@@ -25,7 +25,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--reference-dir", default=os.path.join(ROOT, "baseline", "_ref"))
+    ap.add_argument("--reference-dir", default=os.path.join(ROOT, "oracle", "_ref"))
     ap.add_argument("--graph-rollout", action="store_true")
     ap.add_argument("--gpu-dyn-graphs", action="store_true")
     ap.add_argument("--seed", type=int, default=None, help="torch.manual_seed / numpy seed before Main.py runs (the reference sets none)")
